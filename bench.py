@@ -62,6 +62,9 @@ def parse():
                     help="untimed rollout steps before the warm-up: all environments start their first episode "
                          "in lock-step (a transient with ~25 %% more work per step, tools/step_series.py); a "
                          "training run lives in the desynchronised steady state reached after ~250 steps")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy "
+                         "(float32); the same arguments give the same inputs, so two builds can be compared")
     return ap.parse_args()
 
 
@@ -473,6 +476,32 @@ def _run_extra_config(torch, dist, name, spec, dev, rank, world, steps, warmup, 
     return out
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_last_step(rollouts, out_dir):
+    """Write what the last device_step returned to its caller: the policy's value / action / log-prob / hidden state
+    and the environment's next observation / reward / not-done mask, from the storage slot that step filled.  Above
+    DUMP_MAX_BYTES a fixed seeded sample of environments is written, their indices in env_index.npy."""
+    import numpy as np
+    import torch
+    s = (rollouts.step - 1) % rollouts.num_steps
+    out = {"value": rollouts.value_preds[s], "action": rollouts.actions[s], "action_log_prob": rollouts.action_log_probs[s],
+           "hidden_state": rollouts.recurrent_hidden_states['human_node_rnn'][s + 1], "reward": rollouts.rewards[s],
+           "not_done": rollouts.masks[s + 1]}
+    out.update({"obs_" + k: v[s + 1] for k, v in rollouts.obs.items()})
+    n = rollouts.rewards.size(1)
+    per_env = sum(4 * v[0].numel() for v in out.values())
+    if per_env * n > DUMP_MAX_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_BYTES // (per_env + 4), replace=False))
+        idx = torch.from_numpy(keep).to(rollouts.rewards.device)
+        out = {k: v.index_select(0, idx) for k, v in out.items()}
+        out["env_index"] = idx
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.float().cpu().numpy())
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -539,6 +568,8 @@ def run_ours(a):
     barrier()
     ms_value = e0.elapsed_time(e1)
     launches = env.launch_count() + eng.launch_count() - l0
+    if a.dump_outputs and rank == 0:
+        dump_last_step(rollouts, a.dump_outputs)
 
     # ---------------------------------------------------------------- e2e: reference-facing API, host round trips
     # pinned staging for the host tensors train.py builds every step (masks / bad_masks / reward): allocated ONCE

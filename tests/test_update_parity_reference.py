@@ -10,8 +10,8 @@ rollout quantities (value_preds, log-probs, hidden) are taken from the fixture.
 Tolerances (fp32, different but algebraically equal association: folded projections, compacted rows):
 evaluate_actions value / log-prob / entropy <= 1e-5 relative to the tensor's scale; losses 1e-5 relative;
 post-update parameters: per-tensor sums to 1e-6 relative of the abs-sum, leading entries 2e-6 absolute
-(the Adam step is lr = 4e-5 per entry, so a wrong-signed or missing gradient moves an entry by >= 4e-5).
-When /root/reference is present the live reference is run too and EVERY parameter entry is compared."""
+(the Adam step is lr = 4e-5 per entry, so a wrong-signed or missing gradient moves an entry by >= 4e-5);
+single entries of a seeded sample of every tensor 1e-6 absolute (tests/golden/update_t30_n8_entries.npz)."""
 import os
 import sys
 
@@ -20,7 +20,6 @@ import pytest
 import torch
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(REPO, "tools"))
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from policy_fixture import synth_state_dict  # noqa: E402
 
@@ -150,22 +149,22 @@ def test_ppo_update_matches_reference_fixture():
     assert moved >= len(g["param_keys"]) - 3
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/rl/ppo/ppo.py"), reason="live reference only in the build container")
-def test_ppo_update_matches_live_reference_every_entry():
-    import make_golden_update as mg
-    out, ref_pol = mg.run_reference()
+def test_ppo_update_matches_reference_sampled_entries():
+    """Single entries after the update: every entry of the small tensors and a seeded sample of 256 entries of each
+    larger one (tests/golden/update_t30_n8_entries.npz, the reference's post-update minus initial value)."""
     g = _fixture()
-    for k in ("returns", "mb_values", "mb_logp", "losses"):            # the committed fixture is what the reference gives
-        assert np.allclose(out[k], g[k], rtol=1e-6, atol=1e-6), k
+    e = np.load(os.path.join(REPO, "tests", "golden", "update_t30_n8_entries.npz"))
     pol, losses = _mirror_update(g)
-    ref_sd, sd = ref_pol.state_dict(), pol.state_dict()
+    sd = pol.state_dict()
     pre = synth_state_dict(sd)
+    assert sorted(sd.keys()) == [str(k) for k in e["param_keys"]]
     worst = 0.0
-    for k in ref_sd:
-        d_ref = (ref_sd[k] - pre[k]).double()
-        d_own = (sd[k] - pre[k]).double()
-        err = float((d_ref - d_own).abs().max())
+    for i, k in enumerate(e["param_keys"]):
+        k, sel = str(k), e["tensor"] == i
+        d_ref = e["delta"][sel].astype(np.float64)
+        d_own = (sd[k] - pre[k]).reshape(-1).numpy()[e["index"][sel]].astype(np.float64)
+        err = float(np.abs(d_ref - d_own).max())
         worst = max(worst, err)
         # 4 Adam steps of lr 4e-5: |delta| <= 1.6e-4 per entry; agreement to 2 % of ONE step
-        assert err <= 1e-6, (k, err, float(d_ref.abs().max()))
-    print("max |delta_ref - delta_own| over all 2.5M entries:", worst)
+        assert err <= 1e-6, (k, err, float(np.abs(d_ref).max()))
+    print("max |delta_ref - delta_own| over %d sampled entries:" % len(e["delta"]), worst)

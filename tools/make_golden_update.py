@@ -9,15 +9,18 @@ environments, chosen so that episodes end mid-rollout), teacher-forced through t
 into the reference RolloutStorage, then: compute_returns (GAE), recurrent_generator under a fixed torch seed,
 evaluate_actions on the first minibatch and ONE PPO.update (2 epochs x 2 minibatches, entropy_coef != 0 so the
 entropy term is pinned).  Stored: the rollout inputs, returns, the minibatch outputs, the three losses and, per
-parameter tensor, its sum / abs-sum / first 4 entries after the update (the full 10 MB of weights are compared
-live by tests/test_update_parity_reference.py when /root/reference is present).
+parameter tensor, its sum / abs-sum / first 4 entries after the update.  A second file, update_t30_n8_entries.npz,
+holds how the update moved a seeded sample of single entries (every entry of small tensors, ENTRIES_PER_TENSOR of
+each larger one): the full 10 MB of weights are too large to store.
+
+    CROWDNAV_REFERENCE_ROOT=<reference checkout> python tools/make_golden_update.py
 """
 import os
 import sys
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(REPO, "oracle", "shims"))
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["CROWDNAV_REFERENCE_ROOT"])
 sys.path.insert(0, REPO)
 sys.path.insert(0, os.path.join(REPO, "tests"))
 import numpy as np  # noqa: E402
@@ -143,9 +146,34 @@ def run_reference():
     return out, pol
 
 
+ENTRIES_PER_TENSOR = 256
+
+
+def sampled_entries(pol):
+    """Per parameter tensor (sorted keys): flat indices of a seeded sample of its entries and how the update moved
+    each of them (post-update minus synthetic initial value, in fp32)."""
+    from policy_fixture import synth_state_dict
+    sd = pol.state_dict()
+    pre = synth_state_dict(sd)
+    rng = np.random.default_rng(2024)
+    keys, tensor, index, delta = sorted(sd.keys()), [], [], []
+    for i, k in enumerate(keys):
+        n = sd[k].numel()
+        idx = np.arange(n) if n <= ENTRIES_PER_TENSOR else np.sort(rng.choice(n, ENTRIES_PER_TENSOR, replace=False))
+        d = (sd[k] - pre[k]).reshape(-1).numpy()[idx]
+        tensor.append(np.full(len(idx), i, np.int16))
+        index.append(idx.astype(np.int32))
+        delta.append(d.astype(np.float32))
+    return dict(param_keys=np.array(keys), tensor=np.concatenate(tensor), index=np.concatenate(index),
+                delta=np.concatenate(delta))
+
+
 if __name__ == "__main__":
-    out, _ = run_reference()
+    out, pol = run_reference()
     p = os.path.join(REPO, "tests", "golden", "update_t30_n8.npz")
     np.savez_compressed(p, **out)
     print("wrote", p, os.path.getsize(p), "bytes; losses", out["losses"], "entropy", out["mb_entropy"],
           "dones per env", out["done"].sum(0))
+    p = os.path.join(REPO, "tests", "golden", "update_t30_n8_entries.npz")
+    np.savez_compressed(p, **sampled_entries(pol))
+    print("wrote", p, os.path.getsize(p), "bytes")
